@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # B200 path (this repo)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's PyTorch CPU path
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's PCM (DIR/pcm.npy)
 
 One "step" = one pass of the hot path over one batch of utterances per GPU: prefill(500) ->
 250 decode steps (EOS masked until 250, top-k 50 / T=1 sampling on device) -> NeuCodec decode
@@ -48,7 +49,12 @@ def parse():
                     help="fixed: every prompt 500 tokens (configs[1]); mixed: prompt lengths U{200..1400}, seeded (configs[2])")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the batch 8 / 64 lines reported under 'batches' (N=1 runs only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the PCM of the last timed step to DIR/pcm.npy (float32, one row per utterance) to compare builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def peaks():
@@ -306,6 +312,23 @@ def decode_roofline(lm, B, lens, t_dec, n_steps, launches_per_step):
             "us_per_decode_step": t_dec / n_steps * 1e6, "algorithmic_bytes_per_step": sb}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(path, pcm):
+    """PCM of one timed step ([utterances, samples] after the all-gather) -> path/pcm.npy as float32.  The inputs of a
+    step depend only on the arguments (seeded prompts, weights and sampling), so two builds can be compared file for
+    file.  Beyond DUMP_BYTES a fixed, seeded sample of utterances is written, their indices in path/pcm_rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    x = pcm.reshape(-1, pcm.shape[-1]).float().cpu().numpy()
+    keep = (DUMP_BYTES - 256 - 8 * x.shape[0]) // x[0].nbytes     # 256: the two .npy headers
+    if x.shape[0] > keep:
+        rows = np.sort(np.random.default_rng(0).choice(x.shape[0], keep, replace=False))
+        np.save(os.path.join(path, "pcm_rows.npy"), rows.astype(np.float64))
+        x = x[rows]
+    np.save(os.path.join(path, "pcm.npy"), x)
+
+
 def time_decode(lm, prompts, seed=5):
     """(seconds, kernel launches) of the 249-step decode loop alone, CUDA events on the launching stream."""
     sp = lm.sampling(EOS, min_new_tokens=DECODE, max_new_tokens=DECODE, seed=seed)
@@ -486,12 +509,14 @@ def main_b200(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for i in range(args.steps):
-        gather(step_device(100 + i))
+        pcm = gather(step_device(100 + i))
     ev1.record()
     barrier()
     t_dev = ev0.elapsed_time(ev1) / 1e3
     launches = L.nt_launch_count() - n0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pcm)
 
     # the parts, each timed alone with CUDA events
     t_dec, dec_launches = time_decode(lm, prompts)

@@ -1,6 +1,11 @@
 """CPU: the measurement harness's own arithmetic (bench.py) -- workload shape, algorithmic bytes of a decode step,
 the tokenizer stub the end-to-end leg gives the facade, CLI defaults the driver relies on."""
+import os
 import sys
+
+import numpy as np
+import pytest
+import torch
 
 import bench
 from neutts_air_b200.lm import LMShape
@@ -27,3 +32,26 @@ def test_bench_tokenizer_and_cli_defaults(monkeypatch):
     monkeypatch.setattr(sys, "argv", ["bench.py"])
     a = bench.parse()
     assert (a.gpus, a.impl, a.batch) == (1, "b200", 0) and a.warmup >= 3 and a.steps >= 1     # contract: W >= 3, default N = 1
+    assert a.dump_outputs is None
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "7", "--dump-outputs", "out"])
+    a = bench.parse()
+    assert (a.steps, a.dump_outputs) == (7, "out")
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse()
+
+
+def test_dump_outputs_writes_float32_pcm_within_the_budget(tmp_path, monkeypatch):
+    pcm = torch.randn(5, 1, 1000)
+    bench.dump_outputs(str(tmp_path / "a"), pcm)
+    assert sorted(os.listdir(tmp_path / "a")) == ["pcm.npy"]
+    got = np.load(tmp_path / "a" / "pcm.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, pcm[:, 0].numpy())
+    # over the budget: the same seeded subset of utterances every time, indices stored beside it
+    monkeypatch.setattr(bench, "DUMP_BYTES", 3 * 4000 + 40 + 256)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), pcm)
+    rows = np.load(tmp_path / "b" / "pcm_rows.npy")
+    assert rows.dtype == np.float64 and len(rows) == 3 and np.array_equal(rows, np.load(tmp_path / "c" / "pcm_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "b" / "pcm.npy"), pcm[rows.astype(int), 0].numpy())
+    assert sum(f.stat().st_size for f in (tmp_path / "b").iterdir()) <= bench.DUMP_BYTES

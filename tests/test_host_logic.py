@@ -199,8 +199,9 @@ def test_page_pool_and_weight_packing():
     assert pk["lm_head"] is pk["embed"]
 
 
-def test_loader_reads_hf_checkpoint(tmp_path):
+def test_loader_reads_hf_checkpoint(tmp_path, monkeypatch):
     pytest.importorskip("transformers")
+    monkeypatch.setenv("HF_HUB_OFFLINE", "1")        # the missing-repo lookup below stays in the local HF cache
     from neutts_air_b200 import loader
     from neutts_air_b200.lm import LMShape
     from oracle import lm_oracle as LO
@@ -375,25 +376,26 @@ def test_reference_signature_defaults():
                    ("codec_repo", "neuphonic/neucodec"), ("codec_device", "cpu")]
 
 
-REF_EXAMPLE = "/root/reference/examples/basic_example.py"
+EXAMPLE_CALLS = os.path.join(os.path.dirname(__file__), "golden", "basic_example_calls.json")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_EXAMPLE), reason="reference checkout not mounted (GPU box)")
 def test_reference_basic_example_runs_unmodified(tmp_path, monkeypatch):
-    """SURVEY §8c golden (4): the reference's examples/basic_example.py, imported as it is, drives THIS repo's
+    """SURVEY §8c golden (4): the calls the reference's examples/basic_example.py makes when it runs unmodified
+    (recorded by oracle/record_example_calls.py into tests/golden/basic_example_calls.json) drive THIS repo's
     ``neutts.NeuTTS`` (ctor with the reference's device strings, encode_reference, infer, soundfile.write) and
-    writes a wav of 480 * N samples.  Checkpoints, tokenizer and espeak do not exist offline, so the three loaders
-    are replaced by the fakes of this file; everything else -- the example and the facade -- runs unmodified."""
-    import importlib.util
-    import sys
-    import types
+    write a wav of 480 * N samples.  Checkpoints, tokenizer and espeak do not exist offline, so the three loaders
+    are replaced by the fakes of this file; the facade runs unmodified."""
+    import importlib
 
     import neutts.neutts as NN
 
+    trace = json.load(open(EXAMPLE_CALLS))
+    assert [c["call"] for c in trace["calls"]] == ["neutts.NeuTTS", "NeuTTS.encode_reference", "NeuTTS.infer", "soundfile.write"]
     written = {}
-    sf = types.ModuleType("soundfile")
-    sf.write = lambda path, wav, sr: written.update(path=path, wav=np.asarray(wav), sr=sr)
-    monkeypatch.setitem(sys.modules, "soundfile", sf)
+
+    def sf_write(path, wav, sr):
+        written.update(path=path, wav=np.asarray(wav), sr=sr)
+
     tok = FakeTokenizer()
     tail = [tok.speech_base + c for c in (5, 9, 11, 70000, 13)] + [65, tok.special_base + 5]   # 4 valid codes, junk, EOS
     seen = {}
@@ -413,16 +415,29 @@ def test_reference_basic_example_runs_unmodified(tmp_path, monkeypatch):
     # reference voice: audio file + the pre-encoded codes next to it, as the reference ships them (samples/dave.{wav,pt})
     (tmp_path / "dave.wav").write_bytes(b"RIFF....WAVE")
     torch.save(torch.tensor([54, 65493, 7], dtype=torch.int32), tmp_path / "dave.pt")
-    (tmp_path / "dave.txt").write_text("hello there\n")
-    spec = importlib.util.spec_from_file_location("ref_basic_example", REF_EXAMPLE)
-    mod = importlib.util.module_from_spec(spec)
+    for name, text in trace["files"].items():
+        (tmp_path / name).write_text(text)
+    rets = []
+
+    def arg(v):
+        if isinstance(v, dict) and "$ret" in v:
+            return rets[v["$ret"]]
+        return v.replace("{tmp}", str(tmp_path)) if isinstance(v, str) else v
+
     import warnings
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        spec.loader.exec_module(mod)            # `from neutts import NeuTTS` resolves to this repo's package
-        assert mod.NeuTTS is NN.NeuTTS
-        mod.main("Testing.", str(tmp_path / "dave.wav"), str(tmp_path / "dave.txt"), "neuphonic/neutts-air",
-                 output_path=str(tmp_path / "out.wav"))
+        for c in trace["calls"]:
+            args, kwargs = [arg(a) for a in c["args"]], {k: arg(v) for k, v in c["kwargs"].items()}
+            if c["call"] == "neutts.NeuTTS":
+                cls = importlib.import_module("neutts").NeuTTS   # `from neutts import NeuTTS` resolves to this repo's package
+                assert cls is NN.NeuTTS
+                tts = cls(*args, **kwargs)
+                rets.append(tts)
+            elif c["call"] == "soundfile.write":
+                rets.append(sf_write(*args, **kwargs))
+            else:
+                rets.append(getattr(tts, c["call"].split(".", 1)[1])(*args, **kwargs))
     assert seen == {"backbone": ("neuphonic/neutts-air", "cpu"), "codec": ("neuphonic/neucodec", "cpu")}
     assert written["sr"] == 24000 and written["path"].endswith("out.wav")
     assert written["wav"].dtype == np.float32 and written["wav"].shape == (480 * 4,) and np.isfinite(written["wav"]).all()
