@@ -216,8 +216,15 @@ size_t nt_codec_workspace_bytes(const nt_codec_config* cfg);
 int nt_codec_create(const nt_codec_config* cfg, const nt_codec_weights* w, void* workspace, size_t workspace_bytes,
                     nt_codec** out);
 int nt_codec_destroy(nt_codec* c);
-/* codes: device int32 [B][N] (all items the same length N); pcm: device f32 [B][hop*N]. */
+/* codes: device int32 [B][N] (all items the same length N); pcm: device f32 [B][hop*N].
+ * The same forward pass as nt_codec_decode_ragged with every length N. */
 int nt_codec_decode(nt_codec* c, const int32_t* codes, int B, int N, float* pcm, void* stream);
+/* Items of different lengths in one forward pass.
+ * codes: device int32, items packed back to back: item b = codes[cu_frames[b] .. cu_frames[b+1]);
+ * cu_frames: HOST int32 [B+1], cu_frames[0] = 0, every length in 1..max_frames, 1 <= B <= max_batch;
+ * pcm: device f32 [hop * cu_frames[B]], item b at pcm[hop*cu_frames[b]] (hop*N_b samples).
+ * Asynchronous on `stream` (no host synchronisation); item b's samples equal a decode of item b alone. */
+int nt_codec_decode_ragged(nt_codec* c, const int32_t* codes, const int32_t* cu_frames, int B, float* pcm, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Single-op entry points (unit tests; each mirrors one row of SURVEY.md §8a)

@@ -31,6 +31,12 @@ SPEECH_RE = re.compile(r"<\|speech_(\d+)\|>")
 CHAT = "user: Convert the text to speech:<|TEXT_REPLACE|>\nassistant:<|SPEECH_REPLACE|>"
 
 
+def _split_frames(pcm: np.ndarray, lengths: Sequence[int]) -> list:
+    """Packed PCM of a ragged codec call -> one waveform per item (hop = samples per frame)."""
+    hop = pcm.shape[-1] // sum(lengths)
+    return np.split(pcm, np.cumsum([hop * n for n in lengths])[:-1])
+
+
 class _CrossFade:
     """Incremental equivalent of the reference's ``_linear_overlap_add`` (``neutts/neutts.py:46-70``):
     triangular weights over every chunk, weighted sum / weight sum, but only the samples a new chunk
@@ -220,7 +226,9 @@ class NeuTTS:
 
     # ------------------------------------------------------------------ hot path B
     def _decode_codes(self, codes: Sequence[torch.Tensor]) -> list:
-        """codes: list of 1-D int tensors -> list of float32 numpy waveforms (batched by equal length)."""
+        """codes: list of 1-D int tensors -> list of float32 numpy waveforms.  A codec with ``decode_code_ragged`` takes
+        up to ``max_batch`` utterances per call in input order, whatever their lengths; any other codec gets one
+        ``decode_code`` call per distinct length."""
         out = [None] * len(codes)
         by_len: dict = {}
         for i, c in enumerate(codes):
@@ -228,6 +236,14 @@ class NeuTTS:
                 raise ValueError("No valid speech tokens found in the output.")
             by_len.setdefault(len(c), []).append(i)
         cap = getattr(self.codec, "max_batch", 1)
+        if hasattr(self.codec, "decode_code_ragged"):
+            for j in range(0, len(codes), cap):
+                grp = [codes[i].long().flatten() for i in range(j, min(j + cap, len(codes)))]
+                lens = [len(c) for c in grp]
+                with torch.no_grad():
+                    pcm = self.codec.decode_code_ragged(torch.cat(grp).to(self.codec.device), lens).cpu().numpy()
+                out[j: j + len(grp)] = _split_frames(pcm, lens)
+            return out
         for n, idxs in by_len.items():
             for j in range(0, len(idxs), cap):
                 grp = idxs[j: j + cap]
@@ -358,24 +374,36 @@ class NeuTTS:
             absorbed.copy_(torch.minimum(ngen, torch.full_like(ngen, hi)))
 
         def decode_windows(jobs):
-            """jobs: (slot, t0, t1, s0, s1 | None).  Same-length windows share one codec call."""
-            out = {}
-            by_len = {}
-            for j in jobs:
-                by_len.setdefault(j[2] - j[1], []).append(j)
+            """jobs: (slot, t0, t1, s0, s1 | None) -> one waveform slice per job, in job order.  A codec with
+            ``decode_code_ragged`` takes every window of the round in calls of at most ``max_batch``, gathered from the
+            history with one flat index; any other codec gets one ``decode_code`` call per window length."""
+            out = [None] * len(jobs)
             cbatch = max(1, getattr(self.codec, "max_batch", 1))
-            for n, grp in by_len.items():
-                for g0 in range(0, len(grp), cbatch):
-                    g = grp[g0: g0 + cbatch]
-                    rows = torch.tensor([j[0] for j in g], device=dev)
-                    idx = torch.tensor([j[1] for j in g], device=dev)[:, None] + torch.arange(n, device=dev)[None, :]
-                    codes = hist[rows[:, None], idx][:, None, :]
-                    with torch.no_grad():
-                        pcm = self.codec.decode_code(codes.to(self.codec.device))
-                    pcm = pcm[:, 0, :].cpu().numpy()
-                    for r, (b, t0, t1, s0, s1) in enumerate(g):
-                        wav = self._watermark(pcm[r])
-                        out.setdefault(b, []).append(wav[max(s0, 0):] if s1 is None else wav[s0:s1])
+            ragged = hasattr(self.codec, "decode_code_ragged")
+            if ragged:
+                groups = [list(range(g0, min(g0 + cbatch, len(jobs)))) for g0 in range(0, len(jobs), cbatch)]
+            else:
+                by_len = {}
+                for i, j in enumerate(jobs):
+                    by_len.setdefault(j[2] - j[1], []).append(i)
+                groups = [g[g0: g0 + cbatch] for g in by_len.values() for g0 in range(0, len(g), cbatch)]
+            for g in groups:
+                lens = [jobs[i][2] - jobs[i][1] for i in g]
+                with torch.no_grad():
+                    if ragged:
+                        flat = torch.cat([torch.arange(jobs[i][0] * (cap + 1) + jobs[i][1], jobs[i][0] * (cap + 1) + jobs[i][2])
+                                          for i in g])
+                        codes = hist.view(-1)[flat.to(dev)]
+                        wavs = _split_frames(self.codec.decode_code_ragged(codes.to(self.codec.device), lens).cpu().numpy(), lens)
+                    else:
+                        rows = torch.tensor([jobs[i][0] for i in g], device=dev)
+                        idx = torch.tensor([jobs[i][1] for i in g], device=dev)[:, None] + torch.arange(lens[0], device=dev)[None, :]
+                        codes = hist[rows[:, None], idx][:, None, :]
+                        wavs = list(self.codec.decode_code(codes.to(self.codec.device))[:, 0, :].cpu().numpy())
+                for i, pcm in zip(g, wavs):
+                    s0, s1 = jobs[i][3], jobs[i][4]
+                    wav = self._watermark(pcm)
+                    out[i] = wav[max(s0, 0):] if s1 is None else wav[s0:s1]
             return out
 
         lm.prefill(prompts, sp)             # samples the first token of every slot
@@ -395,31 +423,35 @@ class NeuTTS:
                     s0 = (n_dec[b] - t0) * hop
                     jobs.append((b, t0, t1, s0, s0 + (F + 2 * OV) * hop))
                     n_dec[b] += F
-            out = [None] * B
-            if jobs:
-                for b, wavs in decode_windows(jobs).items():
-                    out[b] = np.concatenate([fades[b].push(w) for w in wavs])
-            # ragged tail of a slot that finished (neutts/neutts.py:443-465), once its regular chunks are out
-            tails = []
+            # ragged tail of a slot that finished (neutts/neutts.py:443-465), once its regular chunks are out; the
+            # tails go through the codec together with this round's regular windows
+            has_chunk = {j[0] for j in jobs}
+            tails, flushes = [], []
             all_finished = all(finished)
             for b in range(B):
-                if finished[b] and not tail_done[b] and (all_finished or out[b] is None):
+                if finished[b] and not tail_done[b] and (all_finished or b not in has_chunk):
                     tail_done[b] = True
                     n = int(hlen_h[b])
                     if n > n_dec[b]:
                         rem = n - n_dec[b]
                         t0 = max(n - (LB + OV + rem), 0)
                         tails.append((b, t0, n, (n - t0 - rem - OV) * hop, None))
-                    elif fades[b].acc.shape[0]:
-                        flush = fades[b].push(np.zeros(0, np.float32), final=True)
-                        out[b] = flush if out[b] is None else np.concatenate((out[b], flush))
+                    else:
+                        flushes.append(b)
+            wavs = decode_windows(jobs + tails) if jobs or tails else []
+            out = [None] * B
+            for b in sorted(has_chunk):
+                out[b] = np.concatenate([fades[b].push(w) for j, w in zip(jobs, wavs) if j[0] == b])
+            for b in flushes:
+                if fades[b].acc.shape[0]:
+                    flush = fades[b].push(np.zeros(0, np.float32), final=True)
+                    out[b] = flush if out[b] is None else np.concatenate((out[b], flush))
             if all_finished and any(o is not None for o in out) and tails:
                 yield out                    # regular chunks first: a tail is its own yield, as in the reference
                 out = [None] * B
-            if tails:
-                for b, wavs in decode_windows(tails).items():
-                    t = fades[b].push(wavs[0], final=True)
-                    out[b] = t if out[b] is None else np.concatenate((out[b], t))
+            for (b, *_), w in zip(tails, wavs[len(jobs):]):
+                t = fades[b].push(w, final=True)
+                out[b] = t if out[b] is None else np.concatenate((out[b], t))
             if any(o is not None for o in out):
                 yield out
             if all_finished:

@@ -91,6 +91,7 @@ EXPORTS = [
     "nt_lm_workspace_bytes", "nt_lm_create", "nt_lm_destroy", "nt_lm_prefill", "nt_lm_decode", "nt_lm_head_gemv",
     "nt_lm_debug_set_layers", "nt_lm_debug_ptr", "nt_lm_debug_set_profile", "nt_debug_launch_chain",
     "nt_codec_workspace_bytes", "nt_codec_create", "nt_codec_destroy", "nt_codec_decode",
+    "nt_codec_decode_ragged",
     "nt_op_rmsnorm", "nt_op_topk_sample",
 ]
 
@@ -132,6 +133,7 @@ def lib() -> C.CDLL:
     L.nt_codec_create.argtypes = [C.POINTER(CodecConfig), C.POINTER(CodecWeights), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]
     L.nt_codec_destroy.argtypes = [C.c_void_p]
     L.nt_codec_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+    L.nt_codec_decode_ragged.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p, C.c_void_p]
     L.nt_op_rmsnorm.argtypes = [C.c_void_p, C.c_void_p, C.c_float, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     L.nt_op_topk_sample.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(Sampling), C.c_void_p, C.c_int32,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]

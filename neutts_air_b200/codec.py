@@ -4,7 +4,9 @@
 from __future__ import annotations
 
 import ctypes as C
+import itertools
 import math
+from collections.abc import Sequence
 from dataclasses import dataclass
 
 import torch
@@ -155,6 +157,37 @@ class CodecDecoder:
             c32 = codes[:, 0, :].to(self.device, torch.int32).contiguous()
             pcm = torch.empty(B, 1, self.shape.hop * N, dtype=torch.float32, device=self.device)
             _lib.check(self.L.nt_codec_decode(self.handle, c32.data_ptr(), B, N, pcm.data_ptr(), _lib.current_stream_ptr()))
+        return pcm
+
+    @torch.no_grad()
+    def decode_code_ragged(self, codes: torch.Tensor, lengths: Sequence[int], validate: bool | None = None) -> torch.Tensor:
+        """Items of different lengths in one codec pass.  codes: integer [T], the items packed back to back (item b =
+        codes[sum(lengths[:b]) : sum(lengths[:b+1])]) -> float32 [hop*T] on ``self.device``, item b's waveform at
+        [hop*sum(lengths[:b]), hop*sum(lengths[:b+1])).  Each waveform equals ``decode_code`` of that item alone.
+
+        Needs 1..max_batch items of 1..max_frames frames each; id validation follows ``decode_code``."""
+        lengths = [int(n) for n in lengths]
+        if not lengths:
+            raise ValueError("decode_code_ragged needs at least one item")
+        if len(lengths) > self.max_batch:
+            raise ValueError(f"{len(lengths)} items exceed the codec's max_batch {self.max_batch}")
+        if min(lengths) < 1:
+            raise ValueError("No valid speech tokens found in the output.")
+        if max(lengths) > self.max_frames:
+            raise ValueError(f"an item has {max(lengths)} frames, above the codec's max_frames {self.max_frames}")
+        if codes.dim() != 1 or codes.shape[0] != sum(lengths):
+            raise ValueError(f"codes must be 1-D with sum(lengths) = {sum(lengths)} entries, got shape {tuple(codes.shape)}")
+        cmax = self.shape.fsq_levels ** self.shape.fsq_dims
+        if validate is None:
+            validate = codes.device.type == "cpu"
+        if validate and (int(codes.min()) < 0 or int(codes.max()) >= cmax):
+            raise ValueError(f"codec ids must be in [0, {cmax})")
+        cu = (C.c_int32 * (len(lengths) + 1))(0, *itertools.accumulate(lengths))
+        with torch.cuda.device(self.device):
+            c32 = codes.to(self.device, torch.int32).contiguous()
+            pcm = torch.empty(self.shape.hop * codes.shape[0], dtype=torch.float32, device=self.device)
+            _lib.check(self.L.nt_codec_decode_ragged(self.handle, c32.data_ptr(), cu, len(lengths), pcm.data_ptr(),
+                                                     _lib.current_stream_ptr()))
         return pcm
 
     def encode_code(self, audio_or_path):

@@ -1,12 +1,21 @@
 // NeuCodec decoder (seam 2: neutts/neutts.py:288-291 -> codec.decode_code) for sm_100a.
 //
-// Activations are channels-last fp32 in a padded-batch layout: item b owns rows
-// [b*Tp, (b+1)*Tp) with Tp = N + 6; frame t sits at row b*Tp + 3 + t and the 3 rows on either
-// side stay zero, so every Conv1d (k=7 and k=3, "same" padding) is a plain TMA-fed tcgen05
-// GEMM whose K loop walks the taps (gemm_tc.cu) — no im2col buffer, no per-item launches.
+// Activations are channels-last fp32 in a padded-batch layout: item b owns the N_b + 6 rows starting at
+// row0_b = sum_{j<b} (N_j + 6); frame t sits at row row0_b + 3 + t and the 3 rows on either side stay zero, so every
+// Conv1d (k=7 and k=3, "same" padding) is a plain TMA-fed tcgen05 GEMM over all rows whose K loop walks the taps
+// (gemm_tc.cu) -- no im2col buffer, no per-item launches.  Items may have different lengths (nt_codec_decode_ragged);
+// the equal-length nt_codec_decode is the case N_b = N.  Per-item geometry reaches the kernels through a small device
+// table (CodecItem, one async copy per call); kernels over frames run a grid over the longest item and blocks past an
+// item's length return at once.
 // All dense math runs on the tensor cores as TF32 with fp32 accumulation (the <=1e-3 RMS PCM
 // bar of BASELINE.json rules out bf16 operands here); norms, attention softmax, exp/sin/cos
 // and the overlap-add run in fp32 on CUDA cores.
+//
+// Pad rows: only the Conv1d inputs x0 and x2 need zero pad rows, and they are written by fsq_embed_kernel and
+// groupnorm_swish_kernel alone, which touch frame rows only; the per-call memset zeroes the rest.  The GEMMs write every
+// row of their outputs, so pad rows of x1 / x3 / xn / qkv / hbuf / sp / fr carry values no frame row ever reads: every
+// other stage is row-local (row norms, GEMMs without taps, spec_kernel) or reads the frame rows of its own item only
+// (groupnorm, attention, overlap-add).
 //
 // Stage map (SURVEY.md §8a):  B1+B2 fsq_embed_kernel | B3 conv-GEMM | B4 groupnorm_swish_kernel
 // + conv-GEMMs | B5 rmsnorm, GEMMs, rope, codec_attn_kernel | B6 layernorm + head GEMM +
@@ -20,21 +29,28 @@
 
 namespace nt {
 
+// one item of a codec batch: first row of its padded block, frame count, first frame in the packed codes / PCM
+struct CodecItem {
+  int row0, n, frame0, pad_;
+};
+
 // ------------------------------------------------------------------ B1+B2: codes -> fc_post_a(project_out(fsq))
-// grid (B*N), 256 threads.  out row = b*Tp + 3 + t.
-__global__ void __launch_bounds__(256) fsq_embed_kernel(const int32_t* codes, int N, int Tp, int C, int levels, int dims,
+// grid (max N, B), 256 threads.  out row = row0_b + 3 + t.
+__global__ void __launch_bounds__(256) fsq_embed_kernel(const int32_t* codes, const CodecItem* items, int C, int levels, int dims,
                                                         const float* w, const float* bias, float* out) {
   pdl_launch_dependents();
   pdl_wait();
-  const int bt = blockIdx.x, b = bt / N, t = bt - b * N;
-  int code = codes[bt];
+  const int t = blockIdx.x;
+  const CodecItem it = items[blockIdx.y];
+  if (t >= it.n) return;
+  int code = codes[it.frame0 + t];
   float z[16];
   const float half = static_cast<float>(levels / 2);
   for (int i = 0; i < dims; ++i) {
     z[i] = (static_cast<float>(code % levels) - half) / half;
     code /= levels;
   }
-  float* o = out + (static_cast<long long>(b) * Tp + 3 + t) * C;
+  float* o = out + (static_cast<long long>(it.row0) + 3 + t) * C;
   for (int c = threadIdx.x; c < C; c += 256) {
     float acc = bias[c];
     for (int i = 0; i < dims; ++i) acc += w[c * dims + i] * z[i];
@@ -43,15 +59,17 @@ __global__ void __launch_bounds__(256) fsq_embed_kernel(const int32_t* codes, in
 }
 
 // ------------------------------------------------------------------ B4: GroupNorm + swish
-// grid (groups, B), 256 threads.  cpg = C/groups channels (<= 32) x N frames per group.
-__global__ void __launch_bounds__(256) groupnorm_swish_kernel(const float* x, int N, int Tp, int C, int cpg, float eps,
+// grid (groups, B), 256 threads.  cpg = C/groups channels (<= 32) x N_b frames per group.
+__global__ void __launch_bounds__(256) groupnorm_swish_kernel(const float* x, const CodecItem* items, int C, int cpg, float eps,
                                                               const float* gw, const float* gb, float* out) {
   __shared__ float red[8];
   __shared__ float s_stat;
   pdl_launch_dependents();
   pdl_wait();
-  const int g = blockIdx.x, b = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const long long base = (static_cast<long long>(b) * Tp + 3) * C + g * cpg;
+  const int g = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const CodecItem it = items[blockIdx.y];
+  const int N = it.n;
+  const long long base = (static_cast<long long>(it.row0) + 3) * C + g * cpg;
   const float cnt = static_cast<float>(N) * cpg;
   auto block_sum = [&](float v) {
     v = warp_sum(v);
@@ -116,12 +134,14 @@ __global__ void __launch_bounds__(256) rownorm_kernel(const float* x, int rows, 
 }
 
 // ------------------------------------------------------------------ B5: rotary on q,k (interleaved pairs, frame index)
-// grid (B*N), threads = heads*32 pairs.  qkv row layout: [q(h,d) | k(h,d) | v(h,d)]
-__global__ void codec_rope_kernel(float* qkv, int N, int Tp, int C, int heads, const float* inv_freq) {
+// grid (max N, B), threads = heads*32 pairs; t restarts at 0 in every item.  qkv row layout: [q(h,d) | k(h,d) | v(h,d)]
+__global__ void codec_rope_kernel(float* qkv, const CodecItem* items, int C, int heads, const float* inv_freq) {
   pdl_launch_dependents();
   pdl_wait();
-  const int bt = blockIdx.x, b = bt / N, t = bt - b * N;
-  float* row = qkv + (static_cast<long long>(b) * Tp + 3 + t) * 3 * C;
+  const int t = blockIdx.x;
+  const CodecItem it = items[blockIdx.y];
+  if (t >= it.n) return;
+  float* row = qkv + (static_cast<long long>(it.row0) + 3 + t) * 3 * C;
   for (int i = threadIdx.x; i < heads * 32; i += blockDim.x) {
     const int h = i >> 5, pr = i & 31;
     float s, c;
@@ -136,16 +156,20 @@ __global__ void codec_rope_kernel(float* qkv, int N, int Tp, int C, int heads, c
 }
 
 // ------------------------------------------------------------------ B5: bidirectional attention, fp32
-// grid (ceil(N/128), heads, B), 128 threads; thread = one query row; K/V tiles of 32 frames in smem.
-__global__ void __launch_bounds__(128) codec_attn_kernel(const float* qkv, int N, int Tp, int C, float scale_log2, float* out) {
+// grid (ceil(max N/128), heads, B), 128 threads; thread = one query row; K/V tiles of 32 frames in smem.
+// Blocks past the item's length return before the first __syncthreads (the exit is block-uniform).
+__global__ void __launch_bounds__(128) codec_attn_kernel(const float* qkv, const CodecItem* items, int C, float scale_log2, float* out) {
   __shared__ __align__(16) float sK[32 * 64];
   __shared__ __align__(16) float sV[32 * 64];
   pdl_launch_dependents();
   pdl_wait();
-  const int qb = blockIdx.x, h = blockIdx.y, b = blockIdx.z, tid = threadIdx.x;
+  const int qb = blockIdx.x, h = blockIdx.y, tid = threadIdx.x;
+  const CodecItem it = items[blockIdx.z];
+  const int N = it.n;
+  if (qb * 128 >= N) return;
   const int tq = qb * 128 + tid;
   const bool active = tq < N;
-  const long long row0 = static_cast<long long>(b) * Tp + 3;
+  const long long row0 = static_cast<long long>(it.row0) + 3;
   float q[64], o[64], m = -INFINITY, l = 0.f;
   if (active) {
     const float4* qp = reinterpret_cast<const float4*>(qkv + (row0 + tq) * 3 * C + h * 64);
@@ -230,10 +254,12 @@ __global__ void spec_kernel(float* sp, long long ld, int nb, float clip) {
 
 // ------------------------------------------------------------------ B7: overlap-add + envelope ("same" padding)
 // frames rows already carry the synthesis window (folded into the inverse-rDFT basis).
-__global__ void __launch_bounds__(256) ola_kernel(const float* frames, int N, int Tp, int n_fft, int hop, float* pcm) {
+// grid (ceil(hop * max N / 256), B); item b's hop*N_b samples start at pcm[hop * frame0_b].
+__global__ void __launch_bounds__(256) ola_kernel(const float* frames, const CodecItem* items, int n_fft, int hop, float* pcm) {
   pdl_launch_dependents();
   pdl_wait();
-  const int b = blockIdx.y;
+  const CodecItem it = items[blockIdx.y];
+  const int N = it.n;
   const int n = blockIdx.x * 256 + threadIdx.x;
   const int total = hop * N;
   if (n >= total) return;
@@ -246,11 +272,11 @@ __global__ void __launch_bounds__(256) ola_kernel(const float* frames, int N, in
   for (int t = t_hi; t >= 0; --t) {
     const int m = np - t * hop;
     if (m >= n_fft) break;
-    acc += frames[(static_cast<long long>(b) * Tp + 3 + t) * n_fft + m];
+    acc += frames[(static_cast<long long>(it.row0) + 3 + t) * n_fft + m];
     const float w = 0.5f * (1.0f - cosf(w0 * static_cast<float>(m)));
     env += w * w;
   }
-  pcm[static_cast<long long>(b) * total + n] = acc / env;
+  pcm[static_cast<long long>(hop) * it.frame0 + n] = acc / env;
 }
 
 // 3xTF32 operand split: hi = x rounded to the 10-bit TF32 mantissa (exactly representable, so the tensor core's own
@@ -282,6 +308,7 @@ struct nt_codec {
   nt_codec_weights w;
   std::vector<const float*> rn[8], blk[6];
   float *x0, *x1, *x2, *x3, *xn, *qkv, *hbuf, *att, *sp, *fr, *inv_freq;
+  CodecItem* items;   // [max_batch] geometry of the current call's items (filled by one async copy per call)
   int kpad;
   // 3xTF32 (cfg.precision != 1): split weights, split-activation scratch, partial-sum scratch
   SplitW s_head, s_idft, s_embed;
@@ -318,6 +345,7 @@ static size_t codec_carve(const nt_codec_config& c, void* ws, size_t bytes, nt_c
   k->sp = a.take<float>(rows * kpad);
   k->fr = a.take<float>(rows * c.n_fft);
   k->inv_freq = a.take<float>(64);
+  k->items = a.take<CodecItem>(c.max_batch);
   if (c.precision != 1) {
     const size_t C = c.hidden, nb2 = size_t(c.n_fft) + 2;
     auto takew = [&](SplitW& w, size_t rows_, size_t ld) {   // one block: hi rows, then lo rows
@@ -418,11 +446,12 @@ extern "C" int nt_codec_destroy(nt_codec* c) {
 namespace {
 struct CodecRun {
   nt_codec* k;
-  int B, N, Tp, rows, C;
+  int B, maxN, rows, C;
   cudaStream_t s;
 
-  // masked GEMM on the padded layout: out rows r+3 for r with (r % Tp) < N.
-  // A points at the first row the tap window of output row 0 touches.
+  // GEMM on the padded layout.  masked (Conv1d and residual GEMMs): out rows r+3 for r in [0, rows-6), so the tap
+  // window of every output row stays inside the buffer; A points at the first row the window of output row 0 touches.
+  // Rows outside the items' frames are written too and never read (see the header comment).
   // sw (optional): the weight's hi / lo halves -> 3xTF32 in one pass of the GEMM kernel (A_lo.W_hi + A_hi.W_lo +
   // A_hi.W_hi into one TMEM accumulator); the activations are split into a hi / lo pair of buffers first.
   int gemm(const float* A, int K, int lda, const float* W, const float* bias, const float* residual, nt_act act, float* out,
@@ -433,7 +462,6 @@ struct CodecRun {
     a.M = masked ? rows - 6 : rows;
     a.N = Nout, a.K = K, a.A = A, a.lda = lda, a.W = W, a.ldw = ldw ? ldw : K;
     a.bias = bias, a.residual = residual, a.ldr = ldc, a.act = act, a.out_f32 = out, a.ldc = ldc;
-    if (masked) a.valid_period = Tp, a.valid_len = N;
     if (!sw || !sw->hi) return gemm_dispatch(a, s, nullptr, true);
     const int a_rows = a.M + (K + lda - 1) / lda - 1;                      // rows the tap window touches
     const long long a_elems = static_cast<long long>(a_rows) * lda;
@@ -449,35 +477,42 @@ struct CodecRun {
     const nt_codec_config& c = k->cfg;
     const int cpg = C / c.groups;
     int rc;
-    if ((rc = launch_kernel(groupnorm_swish_kernel, dim3(c.groups, B), dim3(256), 0, s, true, (const float*)k->x1, N, Tp, C, cpg,
-                            c.norm_eps, k->rn[0][idx], k->rn[1][idx], k->x2)))
+    if ((rc = launch_kernel(groupnorm_swish_kernel, dim3(c.groups, B), dim3(256), 0, s, true, (const float*)k->x1,
+                            (const CodecItem*)k->items, C, cpg, c.norm_eps, k->rn[0][idx], k->rn[1][idx], k->x2)))
       return rc;
     if ((rc = gemm(k->x2 + 2 * C, 3 * C, C, k->rn[2][idx], k->rn[3][idx], nullptr, NT_ACT_NONE, k->x3 + 3 * C, C, C, true, sp(k->s_rn[0], idx))))
       return rc;
-    if ((rc = launch_kernel(groupnorm_swish_kernel, dim3(c.groups, B), dim3(256), 0, s, true, (const float*)k->x3, N, Tp, C, cpg,
-                            c.norm_eps, k->rn[4][idx], k->rn[5][idx], k->x2)))
+    if ((rc = launch_kernel(groupnorm_swish_kernel, dim3(c.groups, B), dim3(256), 0, s, true, (const float*)k->x3,
+                            (const CodecItem*)k->items, C, cpg, c.norm_eps, k->rn[4][idx], k->rn[5][idx], k->x2)))
       return rc;
     return gemm(k->x2 + 2 * C, 3 * C, C, k->rn[6][idx], k->rn[7][idx], k->x1 + 3 * C, NT_ACT_NONE, k->x1 + 3 * C, C, C, true, sp(k->s_rn[1], idx));
   }
 };
-}  // namespace
 
-extern "C" int nt_codec_decode(nt_codec* k, const int32_t* codes, int B, int N, float* pcm, void* stream_) {
-  if (!k || !codes || !pcm) return set_error(NT_ERR_INVALID, "nt_codec_decode: null argument");
+// One forward pass over B items with frame counts cu_frames[b+1] - cu_frames[b] (host, already validated).
+int codec_forward(nt_codec* k, const int32_t* codes, const int32_t* cu_frames, int B, float* pcm, cudaStream_t s) {
   const nt_codec_config& c = k->cfg;
-  if (B < 1 || B > c.max_batch) return set_error(NT_ERR_INVALID, "codec batch %d not in 1..%d", B, c.max_batch);
-  if (N < 1 || N > c.max_frames) return set_error(NT_ERR_INVALID, "codec frames %d not in 1..%d", N, c.max_frames);
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream_);
-  const int C = c.hidden, Tp = N + 6, rows = B * Tp;
-  CodecRun r{k, B, N, Tp, rows, C, s};
+  std::vector<CodecItem> items(B);
+  int rows = 0, maxN = 0;
+  for (int b = 0; b < B; ++b) {
+    const int n = cu_frames[b + 1] - cu_frames[b];
+    items[b] = CodecItem{rows, n, cu_frames[b], 0};
+    rows += n + 6;
+    if (n > maxN) maxN = n;
+  }
+  const int C = c.hidden;
+  CodecRun r{k, B, maxN, rows, C, s};
   int rc;
+  // the host vector is pageable: the runtime stages it before returning, so it may go out of scope
+  NT_CUDA_CHECK(cudaMemcpyAsync(k->items, items.data(), B * sizeof(CodecItem), cudaMemcpyHostToDevice, s));
+  const CodecItem* it = k->items;
   const size_t act_bytes = size_t(rows + 8) * C * sizeof(float);
   NT_CUDA_CHECK(cudaMemsetAsync(k->x0, 0, act_bytes, s));
   NT_CUDA_CHECK(cudaMemsetAsync(k->x1, 0, act_bytes, s));
   NT_CUDA_CHECK(cudaMemsetAsync(k->x2, 0, act_bytes, s));
 
   // B1+B2
-  if ((rc = launch_kernel(fsq_embed_kernel, dim3(B * N), dim3(256), 0, s, true, codes, N, Tp, C, c.fsq_levels, c.fsq_dims,
+  if ((rc = launch_kernel(fsq_embed_kernel, dim3(maxN, B), dim3(256), 0, s, true, codes, it, C, c.fsq_levels, c.fsq_dims,
                           k->w.fsq_w, k->w.fsq_b, k->x0)))
     return rc;
   // B3: Conv1d k=7 pad=3
@@ -493,9 +528,9 @@ extern "C" int nt_codec_decode(nt_codec* k, const int32_t* codes, int B, int N, 
       return rc;
     if ((rc = r.gemm(k->xn, C, C, k->blk[1][l], nullptr, nullptr, NT_ACT_NONE, k->qkv, 3 * C, 3 * C, false, r.sp(k->s_blk[0], l)))) return rc;
     if (c.rope_time_axis)
-      if ((rc = launch_kernel(codec_rope_kernel, dim3(B * N), dim3(256), 0, s, true, k->qkv, N, Tp, C, c.heads, (const float*)k->inv_freq)))
+      if ((rc = launch_kernel(codec_rope_kernel, dim3(maxN, B), dim3(256), 0, s, true, k->qkv, it, C, c.heads, (const float*)k->inv_freq)))
         return rc;
-    if ((rc = launch_kernel(codec_attn_kernel, dim3((N + 127) / 128, c.heads, B), dim3(128), 0, s, true, (const float*)k->qkv, N, Tp, C,
+    if ((rc = launch_kernel(codec_attn_kernel, dim3((maxN + 127) / 128, c.heads, B), dim3(128), 0, s, true, (const float*)k->qkv, it, C,
                             scale_log2, k->att)))
       return rc;
     if ((rc = r.gemm(k->att + 3 * C, C, C, k->blk[2][l], nullptr, k->x1 + 3 * C, NT_ACT_NONE, k->x1 + 3 * C, C, C, true, r.sp(k->s_blk[1], l))))
@@ -521,5 +556,28 @@ extern "C" int nt_codec_decode(nt_codec* k, const int32_t* codes, int B, int N, 
   if ((rc = launch_kernel(spec_kernel, dim3(rows), dim3(256), 0, s, true, k->sp, (long long)kp, nb, c.mag_clip))) return rc;
   // B7: inverse rDFT (windowed basis) as a GEMM, then overlap-add
   if ((rc = r.gemm(k->sp, 2 * nb, kp, k->w.idft_basis, nullptr, nullptr, NT_ACT_NONE, k->fr, c.n_fft, c.n_fft, false, &k->s_idft, kp))) return rc;
-  return launch_kernel(ola_kernel, dim3((c.hop * N + 255) / 256, B), dim3(256), 0, s, true, (const float*)k->fr, N, Tp, c.n_fft, c.hop, pcm);
+  return launch_kernel(ola_kernel, dim3((c.hop * maxN + 255) / 256, B), dim3(256), 0, s, true, (const float*)k->fr, it, c.n_fft, c.hop, pcm);
+}
+}  // namespace
+
+extern "C" int nt_codec_decode(nt_codec* k, const int32_t* codes, int B, int N, float* pcm, void* stream_) {
+  if (!k || !codes || !pcm) return set_error(NT_ERR_INVALID, "nt_codec_decode: null argument");
+  const nt_codec_config& c = k->cfg;
+  if (B < 1 || B > c.max_batch) return set_error(NT_ERR_INVALID, "codec batch %d not in 1..%d", B, c.max_batch);
+  if (N < 1 || N > c.max_frames) return set_error(NT_ERR_INVALID, "codec frames %d not in 1..%d", N, c.max_frames);
+  std::vector<int32_t> cu(B + 1);
+  for (int b = 0; b <= B; ++b) cu[b] = b * N;
+  return codec_forward(k, codes, cu.data(), B, pcm, reinterpret_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int nt_codec_decode_ragged(nt_codec* k, const int32_t* codes, const int32_t* cu_frames, int B, float* pcm, void* stream_) {
+  if (!k || !codes || !cu_frames || !pcm) return set_error(NT_ERR_INVALID, "nt_codec_decode_ragged: null argument");
+  const nt_codec_config& c = k->cfg;
+  if (B < 1 || B > c.max_batch) return set_error(NT_ERR_INVALID, "codec batch %d not in 1..%d", B, c.max_batch);
+  if (cu_frames[0] != 0) return set_error(NT_ERR_INVALID, "codec cu_frames[0] is %d, must be 0", cu_frames[0]);
+  for (int b = 0; b < B; ++b) {
+    const long long n = static_cast<long long>(cu_frames[b + 1]) - cu_frames[b];
+    if (n < 1 || n > c.max_frames) return set_error(NT_ERR_INVALID, "codec item %d has %lld frames, not in 1..%d", b, n, c.max_frames);
+  }
+  return codec_forward(k, codes, cu_frames, B, pcm, reinterpret_cast<cudaStream_t>(stream_));
 }

@@ -7,6 +7,10 @@
 out=gpurun_out/sanitizer
 mkdir -p $out
 run() { name=$1; shift; timeout 1500 compute-sanitizer "$@" > $out/$name.log 2>&1; echo "rc=$?" >> $out/$name.log; tail -4 $out/$name.log; }
+if [ "$1" = codec_ragged ]; then   # ragged codec batch, tiny config, all three arithmetic modes
+  run memcheck_codec_ragged --tool memcheck --print-limit 20 python -m pytest -q -m gpu tests/test_gpu_codec_ragged.py -k tiny_config
+  exit 0
+fi
 run memcheck_smoke --tool memcheck --print-limit 20 python -c "import __graft_entry__ as g; g.smoke()"
 run memcheck_batched --tool memcheck --print-limit 20 python profiles/sanitizer_batched.py
 run racecheck_smoke --tool racecheck --racecheck-report all --print-limit 20 python -c "import __graft_entry__ as g; g.smoke()"
